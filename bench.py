@@ -2,6 +2,7 @@
 """bench.py -- headline benchmark of the LIBXSMM hot path on B200 (contract: one JSON line on stdout).
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload brgemm|fsspmdm|bcsc|sweep]
+                  [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1]): batched BRGEMM bf16 x bf16 -> f32, m=n=k=64, br=8 (stride mode),
 batch = 65536 independent tiles PER GPU with all operands unique ("mode S" of SURVEY.md 8d). One step is
@@ -13,6 +14,10 @@ one pass over the batch = ONE launch of the tcgen05 tile kernel through the C AB
   roofline      achieved algorithmic GB/s of the dominant kernel vs the measured HBM peak
   cpu_baseline  the reference's own JIT kernel (oracle/_ref, all host cores) on a bounded sample
   also          fsspmdm (config 3) and BCSC (config 4) with their own roofline numbers
+
+--dump-outputs DIR writes the output of the timed path's last step as DIR/<name>.npy (float32), a fixed seeded sample of
+DUMP_CHUNK-element chunks where it is larger than DUMP_BYTES; the inputs are seeded, so two builds can be compared output
+for output.
 
 --impl reference runs the unmodified reference (AMX/AVX-512 JIT through its public dispatch API, OpenMP over
 the batch) on a bounded sample of the same workload on rank 0 only.
@@ -109,6 +114,27 @@ def fill_tenths(t, torch, chunk=1 << 26):
         flat[s:e] = (torch.randint(-5, 6, (e - s,), device=t.device, generator=g, dtype=torch.int8).to(torch.float32) / 10).to(t.dtype)
 
 
+DUMP_BYTES = 16 << 20        # per output; at most four outputs are written, 64 MB in all
+DUMP_CHUNK = 4096
+
+
+def dump_outputs(args, torch, **outs):
+    """the outputs of the timed path (device tensors) as float32 .npy files under args.dump_outputs"""
+    if not args.dump_outputs or int(os.environ.get("RANK", "0")) != 0:
+        return
+    import numpy as np
+    assert len(outs) <= 4
+    os.makedirs(args.dump_outputs, exist_ok=True)
+    for name, t in outs.items():
+        flat = t.reshape(-1)
+        chunks = flat.numel() // DUMP_CHUNK
+        keep = DUMP_BYTES // 4 // DUMP_CHUNK
+        if chunks > keep:
+            idx = np.sort(np.random.default_rng(555).choice(chunks, keep, replace=False))
+            flat = flat[:chunks * DUMP_CHUNK].view(chunks, DUMP_CHUNK)[torch.from_numpy(idx).to(flat.device)]
+        np.save(os.path.join(args.dump_outputs, name + ".npy"), flat.float().cpu().numpy().ravel())
+
+
 def time_steps(torch, fn, steps, warmup, dist=None):
     """W warm-up + K timed steps between barrier+synchronize; CUDA events on the launching stream; max over ranks"""
     for _ in range(warmup):
@@ -196,6 +222,7 @@ def run_ours(args):
             total_ms, per = time_steps(torch, step, args.steps, args.warmup, dist)
         launches = X.libxsmm_b200_launch_count() - launches0 - args.warmup
         X.check()
+        dump_outputs(args, torch, c=c)
         from libxsmm_b200.shard import weak_batch
         per_gpu, job_tiles = weak_batch(BATCH, world)      # batch is the only shard axis: every rank owns BATCH tiles, no collective
         flops = 2.0 * M * N * K * BR * per_gpu
@@ -242,7 +269,7 @@ def run_ours(args):
     elif args.workload == "brgemm_r":
         out = also_brgemm_r(X, torch, pk, args, full=True)
     elif args.workload == "sweep":
-        out = sweep(X, torch, pk, args)
+        out = sweep(X, torch, pk, args, full=True)
     if dist is not None:
         dist.barrier()
         dist.destroy_process_group()
@@ -324,16 +351,19 @@ def also_fsspmdm(X, torch, pk, args, full=False, n_cols=1000000, dist=None):
     one = np.array([1.0], dtype=np.float32); zero = np.array([0.0], dtype=np.float32)
     h = X.libxsmm_fsspmdm_create(F32, Mf, Nf, Kf, Kf, Nf, Nf, one.ctypes.data, zero.ctypes.data, a.ctypes.data, 0, None)
     assert h
-    b = torch.randn(Kf * Nf, device="cuda"); c = torch.empty(Mf * Nf, device="cuda")
+    g = torch.Generator(device="cuda"); g.manual_seed(555)
+    b = torch.randn(Kf * Nf, device="cuda", generator=g); c = torch.empty(Mf * Nf, device="cuda")
     flush = torch.empty(256 << 20, dtype=torch.uint8, device="cuda")
 
     def step():
         X.libxsmm_fsspmdm_execute(h, b.data_ptr(), c.data_ptr())
     step(); X.check()
     checked = fsspmdm_check(torch, a, b, c, Mf, Kf, Nf)
-    steps = max(5, args.steps)
+    steps = args.steps if full else max(5, args.steps)
     total_ms, per = time_steps(torch, step, steps, 3, dist)
     X.check()
+    if full:
+        dump_outputs(args, torch, c=c)
     ms = sorted(per)[len(per) // 2] if dist is None else total_ms / steps
     bytes_alg = 4.0 * (Kf * Nf + Mf * Nf)
     ach = bytes_alg / (ms * 1e-3) / 1e9
@@ -414,9 +444,11 @@ def also_bcsc(X, torch, pk, args, full=False, mblocks=8192, dist=None):
     variant = int(X.libxsmm_b200_bcsc_variant(kernel, nbc))
     assert variant in (1, 2), "BCSC bench did not take a tcgen05 kernel (variant %d)" % variant
     kname = "bcsc_ts_kernel<32,2>" if variant == 2 else "bcsc_tc_kernel<32>"
-    steps = max(3, args.steps // 4)
+    steps = args.steps if full else max(3, args.steps // 4)
     total_ms, per = time_steps(torch, step, steps, 3, dist)
     X.check()
+    if full:
+        dump_outputs(args, torch, c=c)
     ms = sorted(per)[len(per) // 2] if dist is None else total_ms / steps
     bytes_alg = 2.0 * (mblocks * Kb * Mb + mblocks * Nb * Mb) + 2.0 * nnzb * bk * bn
     ach = bytes_alg / (ms * 1e-3) / 1e9
@@ -453,10 +485,10 @@ def sweep_check(torch, a, b, c, m, types, flags, esz, csz, batch):
     return {"tiles": 3, "max_normf_rel": worst, "bit_exact": esz == 1}
 
 
-def sweep(X, torch, pk, args, batch=32768):
+def sweep(X, torch, pk, args, batch=32768, full=False):
     """configs[4]: int8 x int8 -> int32 (U8 x I8, VNNI4 A) and F16 x F16 -> F32, m=n=k in {8..128}, br=1, unique operands"""
     I8, U8, I32, F16 = 12, 13, 8, 3
-    pts = []
+    pts, outs = [], {}
     for name, ta, tb, tcc, tcomp, flags, esz, csz in (("u8*i8->i32", U8, I8, I32, I32, FLAG_BETA_0 | X.GEMM_FLAG_VNNI_A, 1, 4),
                                                        ("f16*f16->f32", F16, F16, F32, F32, FLAG_BETA_0, 2, 4)):
         for m in (8, 16, 32, 64, 128):
@@ -464,10 +496,11 @@ def sweep(X, torch, pk, args, batch=32768):
             kernel = X.libxsmm_dispatch_gemm(shape, flags, 0)
             if not kernel:
                 pts.append({"type": name, "m": m, "error": "dispatch returned NULL"}); continue
-            a = torch.randint(0, 5, (batch * m * m * esz,), dtype=torch.uint8, device="cuda")
-            b = torch.randint(0, 5, (batch * m * m * esz,), dtype=torch.uint8, device="cuda")
+            g = torch.Generator(device="cuda"); g.manual_seed(555 + m)
+            a = torch.randint(0, 5, (batch * m * m * esz,), dtype=torch.uint8, device="cuda", generator=g)
+            b = torch.randint(0, 5, (batch * m * m * esz,), dtype=torch.uint8, device="cuda", generator=g)
             if esz == 2:
-                a = (torch.randint(-5, 6, (batch * m * m,), device="cuda").float() / 10).half(); b = a.roll(7)
+                a = (torch.randint(-5, 6, (batch * m * m,), device="cuda", generator=g).float() / 10).half(); b = a.roll(7)
             c = torch.empty(batch * m * m * csz, dtype=torch.uint8, device="cuda")
             sa = sb = m * m * esz; sc = m * m * csz
 
@@ -476,13 +509,16 @@ def sweep(X, torch, pk, args, batch=32768):
                 assert rc == 0, X.libxsmm_b200_last_error_string()
             step(); X.check()
             chk = sweep_check(torch, a, b, c, m, (ta, tb, tcomp, tcc), flags, esz, csz, batch)
-            total_ms, per = time_steps(torch, step, max(5, args.steps // 2), 3)
+            total_ms, per = time_steps(torch, step, args.steps if full else max(5, args.steps // 2), 3)
             X.check()
+            if full and m == 128:
+                outs[name.split("->")[0].replace("*", "_")] = c.view(torch.int32 if esz == 1 else torch.float32)
             ms = sorted(per)[len(per) // 2]
             bytes_alg = float(batch) * (sa + sb + sc)
             ach = bytes_alg / (ms * 1e-3) / 1e9
             pts.append({"type": name, "m": m, "gflops": 2.0 * m * m * m * batch / (ms * 1e-3) / 1e9, "ms": ms, "gbs": ach, "hbm_frac": ach / pk["hbm_gbs"],
                         "backend": int(X.libxsmm_b200_kernel_backend(kernel)), "oracle_check": chk, "l2_note": "operands %.0f MB%s" % (bytes_alg / 1e6, "" if bytes_alg > 2.5e8 else " (fits L2: not an HBM number)")})
+    dump_outputs(args, torch, **outs)
     best = max((p for p in pts if "gflops" in p), key=lambda p: p["gflops"])
     return {"metric": "mixed-precision sweep GFLOP/s (configs[4], diagonal m=n=k)", "value": best["gflops"], "unit": "GFLOP/s", "n_gpus": 1, "steps": args.steps,
             "warmup": 3, "higher_is_better": True, "dtype": "u8/i8->i32, f16->f32", "data": "synthetic",
@@ -536,8 +572,10 @@ def also_brgemm_r(X, torch, pk, args, full=False, pool_sets=64, batch=BATCH):
         err = gen.normf_rel(gen.to_f64(want, BF16), gen.to_f64(got, BF16))
         assert err <= 5e-3, "mode R output differs from the oracle (tile %d, err %g)" % (t, err)
         worst = max(worst, err)
-    total_ms, per = time_steps(torch, step, max(5, args.steps), 3)
+    total_ms, per = time_steps(torch, step, args.steps if full else max(5, args.steps), 3)
     X.check()
+    if full:
+        dump_outputs(args, torch, c=c)
     ms = sorted(per)[len(per) // 2]
     X.libxsmm_b200_gemm_plan_destroy(plan)
     flops = 2.0 * M * N * K * BR * batch
@@ -786,14 +824,19 @@ def run_reference(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20, help="timed steps (>= 1)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="brgemm", choices=["brgemm", "brgemm_r", "fsspmdm", "bcsc", "sweep"])
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-also", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the timed path's last step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         run_reference(args)

@@ -31,7 +31,6 @@ def test_reference_arm_prints_one_json_line():
         assert j["cpu_baseline"]["cores"] > 1            # OMP_NUM_THREADS=1 from the launcher was overridden
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="oracle/_ref/libxsmm_ref.so not built")
 def test_reference_arm_is_silent_on_other_ranks():
     env = dict(os.environ, RANK="1", WORLD_SIZE="2")
     out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--gpus", "2", "--steps", "1", "--warmup", "0"],

@@ -1,6 +1,6 @@
-"""CPU-only: pins oracle/oracle.c (the restatement) against the UNMODIFIED reference built from
-/root/reference (oracle/_ref/libxsmm_ref.so) on seeded inputs -- bit for bit -- and against the
-reference's JIT path (AMX/AVX-512 on this host) within the reference's own acceptance norms."""
+"""CPU-only: pins oracle/oracle.c (the restatement) against the UNMODIFIED reference (oracle/_ref/libxsmm_ref.so)
+on seeded inputs -- bit for bit -- and against the reference's JIT path (AMX/AVX-512) within the reference's own
+acceptance norms. Where the reference is not built, its stored answers stand in for it (tests/ref_answers.py)."""
 import ctypes as C
 
 import numpy as np
@@ -8,53 +8,51 @@ import pytest
 
 import cases
 import gen
+import ref_answers as R
 from oracle_ffi import iarr, oracle, ref, run_gemm
 
-needs_ref = pytest.mark.skipif(ref is None, reason="oracle/_ref/libxsmm_ref.so not built (no /root/reference here)")
 
-
-@needs_ref
 def test_conversions_match_reference():
     rng = np.random.default_rng(1)
     bits = np.concatenate([rng.integers(0, 2**32, size=20000, dtype=np.uint64).astype(np.uint32),
                            np.array([0, 0x80000000, 0x7f800000, 0xff800000, 0x7fc00000, 0x7f800001, 0x00000001, 0x007fffff,
                                      0x38800000, 0x387fffff, 0x33000000, 0x33000001, 0x477fe000, 0x477ff000, 0x47800000], dtype=np.uint32)])
-    for u in bits:
-        f = float(np.array([u], dtype=np.uint32).view(np.float32)[0])
-        assert oracle["f32_to_bf16"](f) == ref["f32_to_bf16"](f), hex(u)
-        assert oracle["f32_to_f16"](f) == ref["f32_to_f16"](f), hex(u)
-    for h in range(0, 65536, 7):
-        a, b = oracle["f16_to_f32"](h), ref["f16_to_f32"](h)
-        assert (a == b) or (a != a and b != b), h
-        a, b = oracle["bf16_to_f32"](h), ref["bf16_to_f32"](h)
-        assert (a == b) or (a != a and b != b), h
+    fs = [float(f) for f in bits.view(np.float32)]
+    for name in ("f32_to_bf16", "f32_to_f16"):
+        R.same(lambda: np.array([ref[name](f) for f in fs], dtype=np.uint16), np.array([oracle[name](f) for f in fs], dtype=np.uint16), name)
+    for name in ("f16_to_f32", "bf16_to_f32"):      # NaN == NaN whatever the payload
+        R.same(lambda: np.array([ref[name](h) for h in range(0, 65536, 7)], dtype=np.float32),
+               np.array([oracle[name](h) for h in range(0, 65536, 7)], dtype=np.float32), name)
 
 
-@needs_ref
 def test_gemm_restatement_is_bit_exact():
     n = 0
     for case in cases.small_cases():
         ops = cases.Operands(case, seed=555 + n)
-        want = cases.ref_result(ref, case, ops, run_gemm)
         got = cases.ref_result(oracle, case, ops, run_gemm)
-        assert np.array_equal(want.view(np.uint8), got.view(np.uint8)), case
+        R.same(lambda: cases.ref_result(ref, case, ops, run_gemm).view(np.uint8), got.view(np.uint8), case)
         n += 1
     assert n > 300
 
 
-@needs_ref
 def test_reference_jit_agrees_with_reference_kernel():
-    """the JIT'ed x86 kernels (the CPU baseline) against the C kernel, reference thresholds (gemm_kernel.c:5312-5414)"""
+    """the JIT'ed x86 kernels (the CPU baseline) against the C kernel, reference thresholds (gemm_kernel.c:5312-5414);
+    the C kernel's answer is the restatement's (bit for bit, test_gemm_restatement_is_bit_exact)"""
     for t, thr in (((gen.F32, gen.F32, gen.F32, gen.F32), 1.2e-5), ((gen.BF16, gen.BF16, gen.F32, gen.F32), 1.2e-5),
                    ((gen.BF16, gen.BF16, gen.F32, gen.BF16), 5e-3), ((gen.U8, gen.I8, gen.I32, gen.I32), 0.0)):
         flags = cases.FLAG_BETA_0 | (cases.FLAG_VNNI_A if t[0] != gen.F32 else 0)
         case = cases.GemmCase(64, 64, 64, *t, flags=flags, br_type=3, br=8)
         ops = cases.Operands(case)
-        c_ref = ops.c0.copy(); c_jit = ops.c0.copy()
-        assert run_gemm(ref, case.dims, case.types, case.flags, 3, ops.stride_a, ops.stride_b, 8, ops.a, ops.b, c_ref, mode=0) == 0
-        rc = run_gemm(ref, case.dims, case.types, case.flags, 3, ops.stride_a, ops.stride_b, 8, ops.a, ops.b, c_jit, mode=1)
-        assert rc in (0, 2)
-        assert gen.normf_rel(gen.to_f64(c_ref, t[3]), gen.to_f64(c_jit, t[3])) <= thr
+        c_ref = ops.c0.copy()
+        assert run_gemm(oracle, case.dims, case.types, case.flags, 3, ops.stride_a, ops.stride_b, 8, ops.a, ops.b, c_ref, mode=0) == 0
+
+        def jit():
+            c_jit = ops.c0.copy()
+            rc = run_gemm(ref, case.dims, case.types, case.flags, 3, ops.stride_a, ops.stride_b, 8, ops.a, ops.b, c_jit, mode=1)
+            assert rc in (0, 2)
+            return gen.to_f64(c_jit, t[3])
+        c_jit, c_ref = R.sampled(jit, gen.to_f64(c_ref, t[3]))
+        assert gen.normf_rel(c_ref, c_jit) <= thr
 
 
 def _bcsc_inputs(rng, ta, tb, tc, mblocks, M, K, N, bk, bn, density, vnni_a=True, trans_a=False):
@@ -77,7 +75,6 @@ def _run_bcsc(side, types, geo, flags, a, bvals, colptr, rowidx, c):
     return side["bcsc"](iarr(*types), iarr(*geo), flags, a.ctypes.data, bvals.ctypes.data, colptr.ctypes.data, rowidx.ctypes.data, c.ctypes.data)
 
 
-@needs_ref
 def test_bcsc_oracle_matches_reference_jit():
     """no portable C kernel exists for BCSC in the reference (no fallback for this build kind): the x86 JIT is
     the second opinion; f32 and bf16 accumulate in a different order, integer paths must agree exactly."""
@@ -89,16 +86,19 @@ def test_bcsc_oracle_matches_reference_jit():
             flags = (cases.FLAG_BETA_0 if beta0 else 0) | (cases.FLAG_VNNI_A if ta != gen.F32 else 0)
             a, bvals, colptr, rowidx, c0 = _bcsc_inputs(rng, ta, tb, tc, mblocks, M, K, N, bk, bn, 0.5)
             geo = (mblocks, M, K, N, bk, bn)
-            c_o, c_r = c0.copy(), c0.copy()
+            c_o = c0.copy()
             assert _run_bcsc(oracle, (ta, tb, tcomp, tc), geo, flags, a, bvals, colptr, rowidx, c_o) == 0
-            rc = _run_bcsc(ref, (ta, tb, tcomp, tc), geo, flags, a, bvals, colptr, rowidx, c_r)
-            if rc != 0:
+
+            def jit():
+                c_r = c0.copy()
+                return gen.to_f64(c_r, tc) if _run_bcsc(ref, (ta, tb, tcomp, tc), geo, flags, a, bvals, colptr, rowidx, c_r) == 0 else None
+            c_r, c_o = R.sampled(jit, gen.to_f64(c_o, tc))
+            if c_r is None:
                 pytest.skip("reference JIT cannot build BCSC for this host ISA")
-            err = gen.normf_rel(gen.to_f64(c_r, tc), gen.to_f64(c_o, tc))
+            err = gen.normf_rel(c_r, c_o)
             assert err <= thr, ((ta, tb, tc), beta0, err)
 
 
-@needs_ref
 def test_fsspmdm_oracle_matches_reference():
     rng = np.random.default_rng(4)
     for dtype, eps in ((gen.F32, 1e-4), (gen.F64, 1e-8)):
@@ -108,23 +108,29 @@ def test_fsspmdm_oracle_matches_reference():
             a = (gen.values(rng, M * K, gen.F64) * (rng.random(M * K) < 0.2)).astype(npdt)
             b = gen.values(rng, K * N, dtype); c0 = gen.values(rng, M * N, dtype)
             alpha = np.array([1.5], dtype=npdt); bt = np.array([beta], dtype=npdt)
-            c_o, c_r = c0.copy(), c0.copy()
+            c_o = c0.copy()
             args = (dtype, M, N, K, K, N, N, alpha.ctypes.data, bt.ctypes.data, a.ctypes.data, b.ctypes.data)
             assert oracle["fsspmdm"](*args, c_o.ctypes.data) == 0
-            assert ref["fsspmdm"](*args, c_r.ctypes.data) == 0
+
+            def run_ref():
+                c_r = c0.copy()
+                assert ref["fsspmdm"](*args, c_r.ctypes.data) == 0
+                return c_r
+            c_r, c_o = R.sampled(run_ref, c_o)
             assert gen.normf_rel(c_r, c_o) <= eps
     # invalid inputs answer "no handle" on both sides (N not a multiple of the vector length, beta=2, empty A)
     M, K, N = 8, 8, 24
     a = np.ones(M * K, dtype=np.float32); b = np.ones(K * N, dtype=np.float32); c = np.zeros(M * N, dtype=np.float32)
     one = np.array([1.0], dtype=np.float32); two = np.array([2.0], dtype=np.float32)
-    for side in (oracle, ref):
-        assert side["fsspmdm"](gen.F32, M, N, K, K, N, N, one.ctypes.data, one.ctypes.data, a.ctypes.data, b.ctypes.data, c.ctypes.data) != 0
-        assert side["fsspmdm"](gen.F32, M, 32, K, K, 32, 32, one.ctypes.data, two.ctypes.data, a.ctypes.data, b.ctypes.data, c.ctypes.data) != 0
-        z = np.zeros(M * K, dtype=np.float32)
-        assert side["fsspmdm"](gen.F32, M, 32, K, K, 32, 32, one.ctypes.data, one.ctypes.data, z.ctypes.data, b.ctypes.data, c.ctypes.data) != 0
+    z = np.zeros(M * K, dtype=np.float32)
+
+    def rcs(side):
+        return np.array([side["fsspmdm"](gen.F32, M, N, K, K, N, N, one.ctypes.data, one.ctypes.data, a.ctypes.data, b.ctypes.data, c.ctypes.data),
+                         side["fsspmdm"](gen.F32, M, 32, K, K, 32, 32, one.ctypes.data, two.ctypes.data, a.ctypes.data, b.ctypes.data, c.ctypes.data),
+                         side["fsspmdm"](gen.F32, M, 32, K, K, 32, 32, one.ctypes.data, one.ctypes.data, z.ctypes.data, b.ctypes.data, c.ctypes.data)])
+    assert np.all(rcs(oracle) != 0) and np.all(R.value(lambda: rcs(ref)) != 0)
 
 
-@needs_ref
 @pytest.mark.parametrize("kind", ["a_csr", "b_csr", "b_csc", "c_csc"])
 def test_packed_sparse_oracle_matches_reference_jit(kind):
     """oracle_packed_sp (restated driver golds, samples/xgemm_norm_packed/*.c) against the reference's own JIT of
@@ -137,25 +143,28 @@ def test_packed_sparse_oracle_matches_reference_jit(kind):
                 is_csc, dims, ptr, idx, a, b, c0 = cases.packed_sp_case(rng, kind, dtype, M, N, K, P)
                 flags = cases.FLAG_BETA_0 if beta0 else 0
                 vals = a if kind == "a_csr" else b if kind.startswith("b_") else c0
-                c_o, c_r = c0.copy(), c0.copy()
+                c_o = c0.copy()
                 args = (is_csc, dtype, iarr(*dims), flags, P, ptr.ctypes.data, idx.ctypes.data, vals.ctypes.data, a.ctypes.data, b.ctypes.data)
                 rc_o = oracle["packed_sp"](*args, c_o.ctypes.data)
-                rc = ref["packed_sp"](*args, c_r.ctypes.data)
                 if kind == "c_csc" and (dtype != gen.F32 or P % 16):
                     assert rc_o != 0          # C-sparse exists for f32 and whole 16-lane vectors only
                     continue
                 assert rc_o == 0
-                if rc != 0:
-                    continue          # the JIT declines this (kind, precision, width) on this host
                 if kind == "c_csc" and beta0:
                     continue          # reference defect: with BETA_0 the 16-accumulator path stores zmm1 while the sums sit in
                                       # zmm0 (..._csc_csparse_avx_avx2_avx512.c:567-590); the oracle overwrites as documented
+
+                def jit():
+                    c_r = c0.copy()
+                    return c_r if ref["packed_sp"](*args, c_r.ctypes.data) == 0 else None
+                c_r, c_o = R.sampled(jit, c_o)
+                if c_r is None:
+                    continue          # the JIT declines this (kind, precision, width) on this host
                 ran += 1
                 assert gen.normf_rel(c_r, c_o) <= eps, (kind, dtype, (M, N, K, P), beta0)
     assert ran > 0, "the reference JIT built none of the cases"
 
 
-@needs_ref
 @pytest.mark.parametrize("types", [(gen.F32, gen.F32, gen.F32, gen.F32), (gen.BF16, gen.BF16, gen.F32, gen.BF16), (gen.BF16, gen.BF16, gen.F32, gen.F32),
                                    (gen.F16, gen.F16, gen.F32, gen.F16)])
 def test_fused_gemm_restatement_matches_reference(types):
@@ -174,13 +183,12 @@ def test_fused_gemm_restatement_matches_reference(types):
                     ops = cases.Operands(case, seed=int(rng.integers(1 << 30)))
                     bias = gen.values(rng, m, tc)
                     mask0 = rng.integers(0, 256, size=((case.ldc + 15) // 16 * 16) // 8 * n + 8, dtype=np.uint8)
-                    outs = []
-                    for side in (ref, oracle):
+
+                    def run(side):
                         c = ops.c0.copy(); mk = mask0.copy()
                         assert cases.run_gemm_ext(side, case, ops, fuse, bias if fuse[0] else None, mk if fuse[2] else None, c) == 0, (case, fuse)
-                        outs.append((c, mk))
-                    assert np.array_equal(outs[0][0].view(np.uint8), outs[1][0].view(np.uint8)), (case, fuse)
-                    assert np.array_equal(outs[0][1], outs[1][1]), (case, fuse, "mask")
+                        return np.concatenate([c.view(np.uint8), mk])      # C, then the mask
+                    R.same(lambda: run(ref), run(oracle), (case, fuse))
 
 
 I4X2 = 18
@@ -197,7 +205,6 @@ def int4_case(rng, m, n, k, br, pad=0):
     return (m, n, k, lda, ldb, ldc), a, b, zpt, c0, blk_a, blk_b
 
 
-@needs_ref
 def test_int4_gemm_restatement_is_bit_exact():
     """U4 x U8 -> I32 with zero points (reference :1273-1321): plain and stride batch-reduce, beta 0/1"""
     rng = np.random.default_rng(90)
@@ -206,11 +213,15 @@ def test_int4_gemm_restatement_is_bit_exact():
             for beta0 in (0, 1):
                 dims, a, b, zpt, c0, blk_a, blk_b = int4_case(rng, m, n, k, br, pad)
                 flags = (cases.FLAG_BETA_0 if beta0 else 0) | cases.FLAG_VNNI_A | FLAG_INTLV_A | (FLAG_MXK_ZPT if br_type else FLAG_COL_VEC_ZPT)
-                c_o, c_r = c0.copy(), c0.copy()
+                c_o = c0.copy()
                 assert oracle["gemm_i4"](iarr(*dims), flags, br_type, blk_a, blk_b, br, a.ctypes.data, b.ctypes.data, c_o.ctypes.data, zpt.ctypes.data) == 0
-                assert ref["gemm_aux"](iarr(*dims), iarr(I4X2, gen.U8, gen.I32, gen.I32), flags, br_type, blk_a, blk_b, br, a.ctypes.data, b.ctypes.data,
-                                       c_r.ctypes.data, 1, zpt.ctypes.data) == 0
-                assert np.array_equal(c_o, c_r), (dims, br_type, beta0)
+
+                def run_ref():
+                    c_r = c0.copy()
+                    assert ref["gemm_aux"](iarr(*dims), iarr(I4X2, gen.U8, gen.I32, gen.I32), flags, br_type, blk_a, blk_b, br, a.ctypes.data, b.ctypes.data,
+                                           c_r.ctypes.data, 1, zpt.ctypes.data) == 0
+                    return c_r
+                R.same(run_ref, c_o, (dims, br_type, beta0))
 
 
 def bitmap_case(rng, m, n, k, ta, tb, tc, density=0.4, pad=0):
@@ -224,7 +235,6 @@ def bitmap_case(rng, m, n, k, ta, tb, tc, density=0.4, pad=0):
     return (m, n, k, m, ldb, ldc), a, b, bitmap, c0
 
 
-@needs_ref
 def test_bitmap_sparse_a_restatement_is_bit_exact():
     """bitmap-compressed A (DECOMPRESS_A_VIA_BITMASK, reference :857-948): F32 and 16-bit operands, beta 0/1"""
     rng = np.random.default_rng(91)
@@ -233,13 +243,17 @@ def test_bitmap_sparse_a_restatement_is_bit_exact():
             for beta0 in (0, 1):
                 dims, a, b, bitmap, c0 = bitmap_case(rng, m, n, k, ta, tb, tc, pad=pad)
                 flags = (cases.FLAG_BETA_0 if beta0 else 0) | FLAG_BITMASK_A | (cases.FLAG_VNNI_A if ta != gen.F32 else 0)
-                c_o, c_r = c0.copy(), c0.copy()
+                c_o = c0.copy()
                 assert oracle["gemm_bitmap"](iarr(*dims), iarr(ta, tb, gen.F32, tc), flags, a.ctypes.data, b.ctypes.data, c_o.ctypes.data, bitmap.ctypes.data) == 0
-                assert ref["gemm_aux"](iarr(*dims), iarr(ta, tb, gen.F32, tc), flags, 0, 0, 0, 1, a.ctypes.data, b.ctypes.data, c_r.ctypes.data, 2, bitmap.ctypes.data) == 0
-                assert np.array_equal(c_o.view(np.uint8), c_r.view(np.uint8)), (dims, (ta, tb, tc), beta0)
+
+                def run_ref():
+                    c_r = c0.copy()
+                    assert ref["gemm_aux"](iarr(*dims), iarr(ta, tb, gen.F32, tc), flags, 0, 0, 0, 1, a.ctypes.data, b.ctypes.data, c_r.ctypes.data, 2,
+                                           bitmap.ctypes.data) == 0
+                    return c_r.view(np.uint8)
+                R.same(run_ref, c_o.view(np.uint8), (dims, (ta, tb, tc), beta0))
 
 
-@needs_ref
 @pytest.mark.parametrize("kind", [0, 1, 2])
 def test_packed_dense_oracle_matches_reference_jit(kind):
     """libxsmm_create_packed_gemm / _ac_rm / _bc_rm (include/libxsmm.h:195-214): restated driver golds against the reference JIT"""
@@ -252,9 +266,14 @@ def test_packed_dense_oracle_matches_reference_jit(kind):
             for beta0 in (0, 1):
                 dims, a, b, c0 = cases.packed_dense_case(rng, kind, dtype, M, N, K, P, pad)
                 flags = cases.FLAG_BETA_0 if beta0 else 0
-                c_o, c_r = c0.copy(), c0.copy()
+                c_o = c0.copy()
                 assert oracle["packed_dense"](kind, dtype, iarr(*dims), flags, P, a.ctypes.data, b.ctypes.data, c_o.ctypes.data) == 0
-                if ref["packed_dense"](kind, dtype, iarr(*dims), flags, P, a.ctypes.data, b.ctypes.data, c_r.ctypes.data) != 0:
+
+                def jit():
+                    c_r = c0.copy()
+                    return c_r if ref["packed_dense"](kind, dtype, iarr(*dims), flags, P, a.ctypes.data, b.ctypes.data, c_r.ctypes.data) == 0 else None
+                c_r, c_o = R.sampled(jit, c_o)
+                if c_r is None:
                     continue
                 ran += 1
                 assert gen.normf_rel(c_r, c_o) <= eps, (kind, dtype, dims, P, beta0)
